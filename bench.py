@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native metering engine (contract: see the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Workload (BASELINE.json `metric`: "audio-samples/sec/GPU (48 kHz stereo, 8192-ch batch) EBU R128 + true-peak"):
@@ -16,6 +16,9 @@ both channels + getters).  One "step" = one such cycle over the whole batch = 16
 `e2e`    = the same cycle through b200m_r128_run_host with pinned HOST buffers, H2D copy and D2H result read inside the
            timed region (PCIe-bound: 64 MiB per cycle cannot shrink, the LV2 contract is float32 audio).
 `--impl reference` times the reference's own CPU code (oracle/_ref, else the oracle port) on every CPU the process may use.
+`--dump-outputs DIR` writes what the headline's last timed step left for its caller (b200m_r128_results on rank 0: the nine
+EBU R128 readings, histogram counts and fragment power of every instance, and the dBTP hold) as DIR/<field>.npy; the input
+ring is seeded, so two builds run with the same arguments can be compared output for output.
 
 The JSON line is printed (and flushed) as soon as the headline, e2e, roofline and cpu_baseline exist; the other BASELINE
 configs, the whole-mix all-reduce and the parity spot check run afterwards and the enriched line is printed again
@@ -181,6 +184,8 @@ def run_b200(args):
     ms = timed_loop(torch, dist, ws, step, K)
     launches = B.launch_count() - l0
     sampler.stop_flag = True; sampler.join()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *bank.results())
     value = ws * SAMPLES_PER_STEP * K / (ms * 1e-3)
     bank.set_precision(B.PREC_EXACT)
     for s in range(W):
@@ -348,6 +353,15 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(d, res, tp):
+    """one .npy per result field (float32; the int32 counts as float64, exactly) plus tp_max.npy: 8192 instances, < 1 MB in all"""
+    os.makedirs(d, exist_ok=True)
+    for name in res.dtype.names:
+        v = res[name]
+        np.save(os.path.join(d, name + ".npy"), v.astype(np.float64 if v.dtype.kind == "i" else np.float32))
+    np.save(os.path.join(d, "tp_max.npy"), tp.astype(np.float32))
+
+
 def spot_check(B, bank, x, blocks_run, ni=2):
     import _oracle as O
     xs = x[:2 * ni].cpu().numpy()
@@ -513,6 +527,7 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=100)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--headline-only", action="store_true", help="skip the other BASELINE configs, whole-mix and spot check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the headline's last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -13,6 +13,23 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with `pytest -m gpu`)")
 
 
+@pytest.hookimpl(hookwrapper=True)
+def pytest_runtest_makereport(item, call):
+    rep = (yield).get_result()
+    if call.when == "call":
+        item.passed_call = rep.passed
+
+
+@pytest.fixture
+def reftape(request):
+    """the reference side of a comparison, live from oracle/_ref or replayed from tests/golden/ref (tests/_reftape.py)"""
+    import _reftape
+    t = _reftape.Tape(request.node.path.stem, request.node.name)
+    yield t
+    if getattr(request.node, "passed_call", False):
+        t.close()
+
+
 def _has_gpu():
     try:
         import torch

@@ -236,7 +236,7 @@ def test_ebur128_plugin_cycle_with_dbtp():
     assert np.isneginf(g2.results()[1]).all()              # dBTP disabled: tp_max = -inf (:365-366)
 
 
-def test_r128_bank_vs_reference_ebur128_plugin():
+def test_r128_bank_vs_reference_ebur128_plugin(reftape):
     """b200m_r128_* against the reference's EBUr128 PLUGIN driven through its own ebur128_run (oracle/_ref compiles
     src/meters.cc unmodified): the nine loudness values and the dBTP hold tp_max must be bit-identical."""
     import torch
@@ -246,11 +246,11 @@ def test_r128_bank_vs_reference_ebur128_plugin():
     x[3] = 0
     xd = torch.from_numpy(x).cuda()
     g = B.EBUr128(n, 48000.0, True); g.control(B.EBUr128.START)
-    o = O.EbuPlugin(n, 48000.0, True)
+    o = reftape.obj(lambda: O.EbuPlugin(n, 48000.0, True))                # replayed from tests/golden/ref without oracle/_ref
     for b in range(140):
         g.run(xd[:, b * 1024:(b + 1) * 1024]); o.run(np.ascontiguousarray(x[:, b * 1024:(b + 1) * 1024]), nthreads=8)
         if b % 20 == 19:
-            res, tp = g.results(); ref = o.read()
+            res, tp = g.results(); ref = reftape.ref(lambda: o.read())
             for i, name in enumerate(RES):
                 assert np.array_equal(res[name].view(np.uint32), ref[:, i].view(np.uint32)), (b, name)
             assert np.array_equal(tp.view(np.uint32), ref[:, 9].view(np.uint32)), (b, tp, ref[:, 9])

@@ -3,7 +3,8 @@ compiled unmodified into oracle/_ref, -DHAVE_LV2_1_8 as every LV2 >= 1.8.1 build
 drives them: the same URID map, the same control-port atom sequences (meteron, metercfg key/value, time:Position), the
 same audio.  After every run() the notify-port buffers must be IDENTICAL BYTES: every radar point, histogram delta,
 ebulevels float and control reply.  The atom wire format itself is restated from the LV2 specification on both sides
-(the SDK is not installed; oracle/lv2stub is the stand-in the reference is compiled against)."""
+(the SDK is not installed; oracle/lv2stub is the stand-in the reference is compiled against).  Without oracle/_ref the
+reference side is replayed from its recording (tests/_reftape.py): notify buffers by length and digest."""
 import ctypes as C
 import struct
 
@@ -11,6 +12,7 @@ import numpy as np
 import pytest
 
 import _oracle as O
+import _reftape as R
 import _signals as S
 from test_lv2_shim_gpu import Feature, _map, descriptors, Plugin
 
@@ -51,12 +53,12 @@ def sequence(events):
     return a
 
 
-def drive(script, nblocks, block=1024, x=None, cap=CAP, rate=48000.0, name="EBUr128", nch=2):
+def drive(t, script, nblocks, block=1024, x=None, cap=CAP, rate=48000.0, name="EBUr128", nch=2):
     """script: {block index: [events]} fed to the control port of both plugins; asserts byte parity of the notify port"""
     import meters_lv2_b200 as B
     mine, l1 = descriptors(B.LIB_PATH)
-    ref, l2 = descriptors(O.PATHS["reference"])
-    g, r = Plugin(mine[name], rate), Plugin(ref[name], rate)
+    ref, l2 = t.obj(lambda: descriptors(O.PATHS["reference"]), 2)
+    g, r = Plugin(mine[name], rate), t.obj(lambda: Plugin(ref[name], rate))
     if x is None:
         x = S.white(2, block * nblocks, seed=17) * np.float32(4.0)
     empty = sequence([])
@@ -75,8 +77,11 @@ def drive(script, nblocks, block=1024, x=None, cap=CAP, rate=48000.0, name="EBUr
             p.run(block)
             size = struct.unpack("<I", note[:4].tobytes())[0]
             outs.append(note[:8 + size].tobytes())
-        assert len(outs[0]) == len(outs[1]), (b, len(outs[0]), len(outs[1]))
-        assert outs[0] == outs[1], (b, next(i for i in range(len(outs[0])) if outs[0][i] != outs[1][i]))
+        rlen = t.ref(lambda: len(outs[1]))
+        assert len(outs[0]) == rlen, (b, len(outs[0]), rlen)
+        if t.live:
+            assert outs[0] == outs[1], (b, next(i for i in range(len(outs[0])) if outs[0][i] != outs[1][i]))
+        assert R.digest(outs[0]) == t.digest(lambda: outs[1]), b
         sizes.append(len(outs[0]))
     g.close(); r.close()
     return sizes
@@ -91,12 +96,12 @@ def test_descriptor_and_missing_urid_map():
     assert not d.contents.instantiate(d, 48000.0, b"", none)               # no urid:map feature -> NULL (:140-144)
 
 
-def test_silent_ui_no_messages():
-    sizes = drive({}, 6)
+def test_silent_ui_no_messages(reftape):
+    sizes = drive(reftape, {}, 6)
     assert set(sizes) == {16}                                               # bare sequence header while the UI is off
 
 
-def test_gui_session_byte_parity():
+def test_gui_session_byte_parity(reftape):
     """UI connects, starts integration with dBTP on, changes radar time, pauses, resets, disconnects."""
     script = {
         1: [obj(MTR + b"meteron")],
@@ -109,11 +114,11 @@ def test_gui_session_byte_parity():
         170: [obj(MTR + b"meteroff")],
         175: [obj(MTR + b"meteron")],                                                  # resync of the stored radar, 16 points per cycle
     }
-    sizes = drive(script, 210)
+    sizes = drive(reftape, script, 210)
     assert max(sizes) > 1500 and sizes[0] == 16
 
 
-def test_transport_follow_and_autoreset():
+def test_transport_follow_and_autoreset(reftape):
     script = {
         0: [obj(MTR + b"meteron"), cfg("TRANSPORTSYNC", 1.0), cfg("AUTORESET", 1.0)],
         5: [position(1.0)],
@@ -122,14 +127,14 @@ def test_transport_follow_and_autoreset():
         50: [cfg("TRANSPORTSYNC", 0.0), position(0.0)],
         60: [cfg("AUTORESET", 0.0), cfg("START", 0)],
     }
-    drive(script, 80)
+    drive(reftape, script, 80)
 
 
-def test_small_notify_buffer_and_odd_blocks():
+def test_small_notify_buffer_and_odd_blocks(reftape):
     """capacity just above the reference's floor: histogram messages are rationed by the space left (:433)"""
     script = {0: [obj(MTR + b"meteron"), cfg("START", 0)]}
-    drive(script, 120, block=1000, cap=1100)
-    drive(script, 40, block=333, cap=4096, rate=44100.0)
+    drive(reftape, script, 120, block=1000, cap=1100)
+    drive(reftape, script, 40, block=333, cap=4096, rate=44100.0)
 
 
 def _levels(buf):
@@ -150,16 +155,22 @@ def _levels(buf):
     return None
 
 
-def test_batched_mode_one_cycle_latency(monkeypatch):
+def _level_bytes(buf, keys):
+    """the 4-byte values of `keys` in the ebulevels object of a notify buffer, concatenated (empty if there is none)"""
+    lv = _levels(buf)
+    return np.frombuffer(b"".join(lv[k] for k in keys), np.uint8) if lv is not None else np.zeros(0, np.uint8)
+
+
+def test_batched_mode_one_cycle_latency(monkeypatch, reftape):
     """B200M_LV2_BATCH: six EBUr128 instances share one bank; what each instance reports in cycle k + 1 is bit for bit what the
     reference plugin reports in cycle k (loudness values, ranges, true peak), with per-instance controls"""
     import meters_lv2_b200 as B
     monkeypatch.setenv("B200M_LV2_BATCH", "6")
     n, nb, blk = 6, 140, 1024
     mine, l1 = descriptors(B.LIB_PATH)
-    ref, l2 = descriptors(O.PATHS["reference"])
+    ref, l2 = reftape.obj(lambda: descriptors(O.PATHS["reference"]), 2)
     gs = [Plugin(mine["EBUr128"]) for _ in range(n)]
-    rs = [Plugin(ref["EBUr128"]) for _ in range(n)]
+    rs = [reftape.obj(lambda: Plugin(ref["EBUr128"])) for _ in range(n)]
     x = S.white(2 * n, blk * nb, seed=61) * np.float32(3.0)
     x[2:4] *= np.float32(0.05)
     keys = [urid(MTR + k) for k in (b"ebu_loudnessM", b"ebu_maxloudnM", b"ebu_loudnessS", b"ebu_maxloudnS", b"ebu_integrated",
@@ -187,12 +198,14 @@ def test_batched_mode_one_cycle_latency(monkeypatch):
                     p.port(2 + 2 * c, bufs[c]); p.port(3 + 2 * c, bufs[c])
                 p.run(blk)
         for i in range(n):
-            lg, lr = _levels(notes_g[i].tobytes()), _levels(notes_r[i].tobytes())
+            lg = _levels(notes_g[i].tobytes())
+            lr = reftape.ref(lambda: _level_bytes(notes_r[i].tobytes(), keys[:8]))
             if lg is not None and prev_ref[i] is not None and b >= 4:
-                for k in keys[:8]:
-                    assert lg[k] == prev_ref[i][k], (b, i, k, struct.unpack("<f", lg[k]), struct.unpack("<f", prev_ref[i][k]))
+                for j, k in enumerate(keys[:8]):
+                    v = prev_ref[i][4 * j:4 * j + 4].tobytes()
+                    assert lg[k] == v, (b, i, k, struct.unpack("<f", lg[k]), struct.unpack("<f", v))
                 checked += 1
-            prev_ref[i] = lr
+            prev_ref[i] = lr if lr.size else None
     assert checked > n * 100
     for p in gs + rs:
         p.close()

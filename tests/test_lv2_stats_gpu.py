@@ -20,7 +20,7 @@ def _audio(n, seed):
     return x
 
 
-def test_bitmeter_windowed_average_reset():
+def test_bitmeter_windowed_average_reset(reftape):
     n, blk = 1024 * 120, 1024
     script = {
         2: [obj(MTR + b"meteron")],
@@ -32,15 +32,15 @@ def test_bitmeter_windowed_average_reset():
         100: [obj(MTR + b"meteroff")],
         110: [obj(MTR + b"meteron"), cfg("RESET", 0)],
     }
-    sizes = drive(script, n // blk, block=blk, x=_audio(n, 5), cap=8192, name="bitmeter", nch=1)
+    sizes = drive(reftape, script, n // blk, block=blk, x=_audio(n, 5), cap=8192, name="bitmeter", nch=1)
     assert max(sizes) > 2400                                 # bim_stats carries the 584-int vector
 
 
-def test_bitmeter_odd_blocks_44k1():
-    drive({0: [obj(MTR + b"meteron")]}, 90, block=441, x=_audio(441 * 90, 6), cap=4096, rate=44100.0, name="bitmeter", nch=1)
+def test_bitmeter_odd_blocks_44k1(reftape):
+    drive(reftape, {0: [obj(MTR + b"meteron")]}, 90, block=441, x=_audio(441 * 90, 6), cap=4096, rate=44100.0, name="bitmeter", nch=1)
 
 
-def test_sigdisthist_session():
+def test_sigdisthist_session(reftape):
     n, blk = 1024 * 100, 1024
     script = {
         1: [obj(MTR + b"meteron")],
@@ -54,9 +54,9 @@ def test_sigdisthist_session():
     }
     x = S.white(2, n, seed=8) * np.float32(0.8)
     x[0, 3000:3100] = 5.0                                    # outside +-1.2: bins beyond the histogram are skipped
-    sizes = drive(script, n // blk, block=blk, x=x, cap=8192, name="SigDistHist", nch=1)
+    sizes = drive(reftape, script, n // blk, block=blk, x=x, cap=8192, name="SigDistHist", nch=1)
     assert max(sizes) > 1500
 
 
-def test_sigdisthist_small_blocks():
-    drive({0: [obj(MTR + b"meteron"), cfg("START", 0)]}, 200, block=64, x=S.white(2, 64 * 200, seed=9), cap=4096, name="SigDistHist", nch=1)
+def test_sigdisthist_small_blocks(reftape):
+    drive(reftape, {0: [obj(MTR + b"meteron"), cfg("START", 0)]}, 200, block=64, x=S.white(2, 64 * 200, seed=9), cap=4096, name="SigDistHist", nch=1)

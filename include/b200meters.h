@@ -204,6 +204,31 @@ int b200m_r128_destroy (b200m_r128* h);
 int b200m_r128_control (b200m_r128* h, int32_t inst, int cmd, void* stream);      /* inst = -1: all */
 int b200m_r128_run_device (b200m_r128* h, const float* d_in, size_t stride, uint32_t nfram, void* stream);
 int b200m_r128_run_host (b200m_r128* h, const float* in, size_t stride, uint32_t nfram);
+/* PCM input: the cycle above on the sample format a decoder, capture card or file reader already holds, converted on the GPU.
+ * fmt = sample type | layout; all types little-endian.  Value handed to the meters (the float32 a host would have passed to
+ * b200m_r128_run_*):
+ *   B200M_PCM_F32  float32                  the bits unchanged (NaN payloads, -0, denormals, +-inf pass through)
+ *   B200M_PCM_S16  int16                    (float)x * 0x1p-15f                                         (exact)
+ *   B200M_PCM_S24  packed 3-byte signed     sign-extended to int32, then (float)x * 0x1p-23f            (exact)
+ *   B200M_PCM_S32  int32                    __int2float_rn (x) * 0x1p-31f: round to nearest even, as the host's (float)x under
+ *                                           the default MXCSR and numpy's astype (np.float32)
+ * Layouts, `stride` counted in elements of the sample type:
+ *   B200M_PCM_PLANAR       channel k = inst*nchan + c starts at element k*stride (the float convention above)
+ *   B200M_PCM_INTERLEAVED  instance inst's frames start at element inst*stride*nchan, sample (f, c) at + f*nchan + c;
+ *                          stride is in frames
+ * Only the alignment of the sample type is assumed (1 byte for S24, 2 for S16, 4 otherwise).  stride >= nfram, 0 < nfram <= 8192.
+ * F32 | PLANAR is b200m_r128_run_device / _run_host itself.  run_device_pcm converts the block on `stream` into a float buffer of
+ * the bank, then runs the cycle on it; run_host_pcm copies the raw PCM bytes (1/2 of the float32 bytes for S16, 3/4 for S24) in
+ * the same instance slices as run_host, and converts each slice on a stream of its own as soon as its copy has landed. */
+enum { B200M_PCM_F32 = 0, B200M_PCM_S16 = 1, B200M_PCM_S24 = 2, B200M_PCM_S32 = 3,
+       B200M_PCM_PLANAR = 0, B200M_PCM_INTERLEAVED = 16 };
+int b200m_r128_run_device_pcm (b200m_r128* h, const void* d_in, uint32_t fmt, size_t stride, uint32_t nfram, void* stream);
+int b200m_r128_run_host_pcm (b200m_r128* h, const void* in, uint32_t fmt, size_t stride, uint32_t nfram);
+/* any bank's device path: a PCM block of n_inst x nchan channels (nchan 1..8; same formats and layouts as above, src_stride in
+ * elements) -> planar float32 rows, row k = inst*nchan + c at d_dst + k*dst_stride (d_dst 16-byte aligned, dst_stride a multiple
+ * of 4 and >= nfram).  Asynchronous on `stream`; the rows then go to any b200m_*_process_device / _run_device. */
+int b200m_pcm_convert (int device, const void* d_src, uint32_t fmt, uint32_t nchan, uint32_t n_inst, size_t src_stride,
+                       uint32_t nfram, float* d_dst, size_t dst_stride, void* stream);
 /* ebu_out: n_inst getter blocks (may be NULL); tp_max_db: n_inst floats, -inf when dBTP is disabled (may be NULL) */
 int b200m_r128_results (b200m_r128* h, b200m_ebu_result* ebu_out, float* tp_max_db, void* stream);
 /* self->dbtp_enable (CTL_UISETTINGS bit 64, src/ebulv2.cc:316-317): the true-peak meters only run while enabled; while

@@ -92,6 +92,9 @@ _PROTOS = {
     "b200m_r128_control": (C.c_int, [_v, C.c_int32, C.c_int, _v]),
     "b200m_r128_run_device": (C.c_int, [_v, _v, C.c_size_t, C.c_uint32, _v]),
     "b200m_r128_run_host": (C.c_int, [_v, _v, C.c_size_t, C.c_uint32]),
+    "b200m_r128_run_device_pcm": (C.c_int, [_v, _v, C.c_uint32, C.c_size_t, C.c_uint32, _v]),
+    "b200m_r128_run_host_pcm": (C.c_int, [_v, _v, C.c_uint32, C.c_size_t, C.c_uint32]),
+    "b200m_pcm_convert": (C.c_int, [C.c_int, _v, C.c_uint32, C.c_uint32, C.c_uint32, C.c_size_t, C.c_uint32, _v, C.c_size_t, _v]),
     "b200m_r128_results": (C.c_int, [_v, _v, _v, _v]),
     "b200m_r128_set_dbtp": (C.c_int, [_v, C.c_int]),
     "b200m_r128_set_precision": (C.c_int, [_v, C.c_int]),
@@ -232,6 +235,63 @@ def _host_planar(x):
         return _np_ptr(x), stride, x.shape[0], x.shape[1]
     assert (not x.is_cuda) and x.dim() == 2 and x.stride(1) == 1
     return C.c_void_p(x.data_ptr()), x.stride(0), x.shape[0], x.shape[1]
+
+
+PCM_F32, PCM_S16, PCM_S24, PCM_S32 = 0, 1, 2, 3
+PCM_PLANAR, PCM_INTERLEAVED = 0, 16
+_PCM_BYTES = {PCM_F32: 4, PCM_S16: 2, PCM_S24: 3, PCM_S32: 4}
+
+
+def _pcm_layout(x, interleaved, nchan):
+    """numpy array or torch tensor of PCM -> (pointer, fmt, stride, nfram, segments, on_device).
+
+    The dtype selects the sample type: float32, int16, int32, or uint8 with a last dimension of 3 (packed little-endian
+    24-bit).  Planar: [rows, nfram] (rows = instances x nchan); interleaved: [instances, nfram, nchan].  Only the outer
+    dimension may be strided; `stride` comes back in elements (planar) or frames (interleaved), as the C ABI counts it."""
+    if isinstance(x, np.ndarray):
+        name, shape, bstrides, ptr, dev = x.dtype.name, x.shape, x.strides, x.ctypes.data, False
+    else:
+        name = str(x.dtype).replace("torch.", "")
+        shape, bstrides, ptr, dev = tuple(x.shape), tuple(s * x.element_size() for s in x.stride()), x.data_ptr(), x.is_cuda
+    types = {"float32": PCM_F32, "int16": PCM_S16, "int32": PCM_S32, "uint8": PCM_S24}
+    if name not in types:
+        raise TypeError("PCM dtype must be float32, int16, int32 or uint8 (packed 24-bit), not %s" % name)
+    t = types[name]
+    bps = _PCM_BYTES[t]
+    if t == PCM_S24:
+        if shape[-1] != 3 or bstrides[-1] != 1:
+            raise ValueError("24-bit PCM is a uint8 array whose last dimension holds the 3 bytes of a sample")
+        shape, bstrides = shape[:-1], bstrides[:-1]
+    inner = (nchan,) if interleaved else ()
+    if len(shape) != 2 + len(inner) or tuple(shape[2:]) != inner:
+        raise ValueError("PCM shape %s: want %s" % (shape, "[instances, nfram, %d]" % nchan if interleaved else "[rows, nfram]"))
+    frame_bytes = bps * (nchan if interleaved else 1)
+    if bstrides[1] != frame_bytes or (interleaved and bstrides[2] != bps):
+        raise ValueError("PCM frames and channels must be contiguous (only the outer dimension may be strided)")
+    nseg, nfram = shape[0], shape[1]
+    stride = bstrides[0] // frame_bytes if nseg > 1 else nfram
+    if nseg > 1 and bstrides[0] % frame_bytes:
+        raise ValueError("PCM row pitch is not a whole number of frames")
+    return ptr, t | (PCM_INTERLEAVED if interleaved else PCM_PLANAR), stride, nfram, nseg, dev
+
+
+def pcm_convert(x, interleaved, nchan=2, out=None, stream=None):
+    """b200m_pcm_convert: a CUDA tensor of PCM (layouts of _pcm_layout) -> planar float32 rows [instances x nchan, nfram]
+    on the same device, the values every bank is fed (the header's conversion table).  `out` may be a row-strided view
+    (16-byte aligned, row stride a multiple of 4)."""
+    import torch
+    p, fmt, stride, nfram, nseg, dev = _pcm_layout(x, interleaved, nchan)
+    if not dev:
+        raise ValueError("pcm_convert takes CUDA tensors; EBUr128.run_pcm takes host arrays")
+    n_inst = nseg if interleaved else nseg // nchan
+    if not interleaved and nseg % nchan:
+        raise ValueError("%d planar rows are not whole instances of %d channels" % (nseg, nchan))
+    if out is None:
+        out = torch.empty((n_inst * nchan, (nfram + 3) & ~3), dtype=torch.float32, device=x.device)[:, :nfram]
+    o, ostride, rows, n = _dev_ptr(out)
+    assert out.dtype == torch.float32 and rows == n_inst * nchan and n == nfram
+    _ck(lib().b200m_pcm_convert(x.device.index or 0, C.c_void_p(p), fmt, nchan, n_inst, stride, nfram, o, ostride, _stream_ptr(stream)))
+    return out
 
 
 def design_ebu(fsamp):
@@ -743,6 +803,21 @@ class EBUr128(_Bank):
             _ck(lib().b200m_r128_run_host(self.h, C.c_void_p(ptr), stride, nfram))
         else:
             _ck(lib().b200m_r128_run_device(self.h, C.c_void_p(ptr), stride, nfram, _stream_ptr(stream)))
+
+    def run_pcm(self, x, interleaved, stream=None):
+        """one cycle on integer or float PCM, converted on the GPU: planar [2N, nfram] or interleaved [N, nfram, 2]; int16,
+        int32, float32, or uint8 [..., 3] for packed 24-bit.  numpy / CPU tensors take the host path, CUDA tensors the device path."""
+        p, fmt, stride, nfram, nseg, dev = _pcm_layout(x, interleaved, 2)
+        assert nseg == (self.n_inst if interleaved else 2 * self.n_inst), "want %d %s" % (
+            self.n_inst if interleaved else 2 * self.n_inst, "instances" if interleaved else "rows")
+        self.run_pcm_ptr(p, fmt, stride, nfram, stream, host=not dev)
+
+    def run_pcm_ptr(self, ptr, fmt, stride, nfram, stream=None, host=False):
+        """b200m_r128_run_host_pcm / _run_device_pcm on a raw pointer; fmt = PCM_{F32,S16,S24,S32} | PCM_{PLANAR,INTERLEAVED}"""
+        if host:
+            _ck(lib().b200m_r128_run_host_pcm(self.h, C.c_void_p(ptr), fmt, stride, nfram))
+        else:
+            _ck(lib().b200m_r128_run_device_pcm(self.h, C.c_void_p(ptr), fmt, stride, nfram, _stream_ptr(stream)))
 
     def results(self, stream=None, out=None, tp=None):
         out = np.empty(self.n_inst, EBU_RESULT_DTYPE) if out is None else out

@@ -20,6 +20,12 @@ extern "C" int ebu_process_sliced (b200m_ebu* h, const float* d_in, size_t strid
                                    int (*after_k1) (void*), void* after_arg);
 int tpk_process_sliced (b200m_tpk* h, const float* d_in, size_t stride, uint32_t nfram, uint32_t tp_mode, cudaStream_t st, int nsl, const uint32_t* bounds, cudaEvent_t* ready,
                         float* r128_tpmax, bool pdl, const void* dr);
+namespace b200m {                     // PCM ingest (pcm.cu)
+int pcm_check_fmt (uint32_t fmt);
+int pcm_sample_bytes (uint32_t fmt);
+int pcm_convert_launch (const void* d_src, uint32_t fmt, uint32_t nchan, uint32_t n_inst, size_t src_stride, uint32_t nfram,
+                        float* d_dst, size_t dst_stride, cudaStream_t st);
+}
 
 using namespace b200m;
 
@@ -34,6 +40,11 @@ struct b200m_r128 {
     cudaStream_t own = nullptr, side = nullptr, copy = nullptr;
     cudaEvent_t ev_tp = nullptr, ev_done = nullptr, ev_ready[R128_SLICES] = {nullptr};
     HostStage stage; bool last_host = false; int concurrent = 1, slices = R128_SLICES;
+    // PCM host path: raw bytes of the block as copied, and the stream that converts slice s once ev_copied[s] has fired,
+    // so that no conversion queues in front of a copy or of an earlier slice's kernels (created on first use)
+    uint8_t* d_raw = nullptr; size_t raw_bytes = 0;
+    cudaStream_t cvt = nullptr;
+    cudaEvent_t ev_copied[R128_SLICES] = {nullptr};
 };
 
 static int env_int (const char* name, int dflt) { const char* v = getenv (name); return v ? atoi (v) : dflt; }
@@ -118,9 +129,13 @@ int b200m_r128_destroy (b200m_r128* h)
     DeviceGuard g (h->device);
     cudaDeviceSynchronize ();
     cudaFree (h->d_tpmax); h->stage.release ();
-    for (cudaStream_t sp : {h->own, h->side, h->copy}) if (sp) cudaStreamDestroy (sp);
+    if (h->d_raw) cudaFree (h->d_raw);
+    for (cudaStream_t sp : {h->own, h->side, h->copy, h->cvt}) if (sp) cudaStreamDestroy (sp);
     for (cudaEvent_t ep : {h->ev_tp, h->ev_done}) if (ep) cudaEventDestroy (ep);
-    for (int s = 0; s < R128_SLICES; ++s) if (h->ev_ready[s]) cudaEventDestroy (h->ev_ready[s]);
+    for (int s = 0; s < R128_SLICES; ++s) {
+        if (h->ev_ready[s]) cudaEventDestroy (h->ev_ready[s]);
+        if (h->ev_copied[s]) cudaEventDestroy (h->ev_copied[s]);
+    }
     delete h;
     return 0;
 }
@@ -182,6 +197,75 @@ int b200m_r128_run_host (b200m_r128* h, const float* in, size_t stride, uint32_t
             B200M_CUDA (cudaMemcpy2DAsync (h->stage.d + r0 * h->stage.cap, h->stage.cap * sizeof (float), in + r0 * stride, stride * sizeof (float),
                                            (size_t)nfram * sizeof (float), r1 - r0, cudaMemcpyHostToDevice, h->copy));
         B200M_CUDA (cudaEventRecord (h->ev_ready[s], h->copy));
+    }
+    h->last_host = true;
+    if (int rc = r128_run (h, h->stage.d, h->stage.cap, nfram, h->own, nsl, h->ev_ready)) return rc;
+    B200M_CUDA (cudaEventRecord (h->ev_done, h->own));
+    return 0;
+}
+
+static int check_pcm_args (b200m_r128* h, const void* in, uint32_t fmt, size_t stride, uint32_t nfram)
+{
+    if (int rc = pcm_check_fmt (fmt)) return rc;
+    if (int rc = check_block_args (h, in, stride, nfram)) return rc;
+    const int bps = pcm_sample_bytes (fmt);
+    if ((uintptr_t)in % (bps == 3 ? 1 : bps)) return set_err (B200M_E_INVAL, "input not aligned to its sample type");
+    return 0;
+}
+
+int b200m_r128_run_device_pcm (b200m_r128* h, const void* d_in, uint32_t fmt, size_t stride, uint32_t nfram, void* stream)
+{
+    if (int rc = check_pcm_args (h, d_in, fmt, stride, nfram)) return rc;
+    if (fmt == (B200M_PCM_F32 | B200M_PCM_PLANAR)) return b200m_r128_run_device (h, (const float*)d_in, stride, nfram, stream);
+    DeviceGuard g (h->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (h->stage.ensure ((size_t)2 * h->n_inst, nfram)) return set_err (B200M_E_NOMEM, "conversion buffer allocation failed");
+    // the float rows reuse the host path's staging buffer: after a host-path cycle, the conversion waits for its kernels
+    if (h->last_host) B200M_CUDA (cudaStreamWaitEvent (st, h->ev_done, 0));
+    h->last_host = false;
+    if (int rc = pcm_convert_launch (d_in, fmt, 2, h->n_inst, stride, nfram, h->stage.d, h->stage.cap, st)) return rc;
+    return r128_run (h, h->stage.d, h->stage.cap, nfram, st, 1, nullptr);
+}
+
+int b200m_r128_run_host_pcm (b200m_r128* h, const void* in, uint32_t fmt, size_t stride, uint32_t nfram)
+{
+    if (int rc = check_pcm_args (h, in, fmt, stride, nfram)) return rc;
+    if (fmt == (B200M_PCM_F32 | B200M_PCM_PLANAR)) return b200m_r128_run_host (h, (const float*)in, stride, nfram);
+    DeviceGuard g (h->device);
+    B200M_ENTER_HOST_PATH (h);
+    const size_t nch = (size_t)2 * h->n_inst;
+    if (h->stage.ensure (nch, nfram)) return set_err (B200M_E_NOMEM, "staging buffer allocation failed");
+    if (!h->cvt) {
+        B200M_CUDA (cudaStreamCreateWithFlags (&h->cvt, cudaStreamNonBlocking));
+        for (int s = 0; s < R128_SLICES; ++s) B200M_CUDA (cudaEventCreateWithFlags (&h->ev_copied[s], cudaEventDisableTiming));
+    }
+    // one segment = a channel row (planar) or the frames of one instance (interleaved); on the device the segments are dense
+    const bool il = (fmt & B200M_PCM_INTERLEAVED) != 0;
+    const size_t bps = (size_t)pcm_sample_bytes (fmt), spi = il ? 1 : 2;          // segments per instance
+    const size_t seg_bytes = (size_t)nfram * bps * (il ? 2 : 1), src_pitch = stride * bps * (il ? 2 : 1);
+    const size_t need = seg_bytes * h->n_inst * spi;
+    if (need > h->raw_bytes) {                                  // grown on demand, never shrunk
+        if (h->d_raw) { B200M_CUDA (cudaStreamSynchronize (h->own)); cudaFree (h->d_raw); h->d_raw = nullptr; h->raw_bytes = 0; }
+        B200M_CUDA (cudaMalloc (&h->d_raw, need));
+        h->raw_bytes = need;
+    }
+    // single buffers, raw and float: the next copy may only start when the previous cycle's conversions and kernels have
+    // read them (ev_done follows both: the kernels of every slice waited for its conversion)
+    if (h->last_host) B200M_CUDA (cudaStreamWaitEvent (h->copy, h->ev_done, 0));
+    const int nsl = h->n_inst >= 64 ? h->slices : 1;
+    for (int s = 0; s < nsl; ++s) {
+        const size_t i0 = (uint64_t)h->n_inst * s / nsl, i1 = (uint64_t)h->n_inst * (s + 1) / nsl;
+        const size_t g0 = i0 * spi, ng = (i1 - i0) * spi;
+        if (stride == nfram)                                    // the host rows are contiguous: one DMA per slice
+            B200M_CUDA (cudaMemcpyAsync (h->d_raw + g0 * seg_bytes, (const uint8_t*)in + g0 * src_pitch, ng * seg_bytes, cudaMemcpyHostToDevice, h->copy));
+        else
+            B200M_CUDA (cudaMemcpy2DAsync (h->d_raw + g0 * seg_bytes, seg_bytes, (const uint8_t*)in + g0 * src_pitch, src_pitch,
+                                           seg_bytes, ng, cudaMemcpyHostToDevice, h->copy));
+        B200M_CUDA (cudaEventRecord (h->ev_copied[s], h->copy));
+        B200M_CUDA (cudaStreamWaitEvent (h->cvt, h->ev_copied[s], 0));
+        if (int rc = pcm_convert_launch (h->d_raw + g0 * seg_bytes, fmt, 2, (uint32_t)(i1 - i0), nfram, nfram,
+                                         h->stage.d + 2 * i0 * h->stage.cap, h->stage.cap, h->cvt)) return rc;
+        B200M_CUDA (cudaEventRecord (h->ev_ready[s], h->cvt));
     }
     h->last_host = true;
     if (int rc = r128_run (h, h->stage.d, h->stage.cap, nfram, h->own, nsl, h->ev_ready)) return rc;
